@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W             # our CUDA path (one rank per GPU via torchrun)
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on the host CPU cores
+    python bench.py --gpus 1 --steps K --dump-outputs DIR     # + loss / gradients of the last timed step as .npy
 
 One step = what CoarseTransformerTrainer.train_step runs (trainer.py:1242-1252): the training wrapper
 `CoarseTransformerWrapper.forward(semantic_token_ids, coarse_token_ids, return_loss=True)` with its defaults
@@ -430,6 +431,32 @@ def gemm_traffic_from_profile():
     return None, None
 
 
+DUMP_GRAD_SAMPLES = 1 << 22  # 16 MB of the ~260 MB fp32 gradient; the whole dump stays far below 64 MB
+
+
+def last_step_outputs(loss, bucket):
+    """what a caller of the timed step gets back: the loss and every parameter's .grad.  The gradients are dumped as
+    one float64 L2 norm per parameter (in model.parameters() order) and the flat fp32 gradient at a fixed, seeded
+    sample of positions, so two builds can be compared element by element without writing all of it."""
+    bucket.sync_views()
+    g = torch.Generator().manual_seed(0)
+    n = min(DUMP_GRAD_SAMPLES, bucket.numel)
+    idx = torch.randint(0, bucket.numel, (n,), generator=g).sort().values.to(bucket.flat.device)
+    norms = torch.stack([torch.linalg.vector_norm(p.grad, dtype=torch.float64) for p in bucket.params])
+    return {"loss": loss.float().cpu().numpy(),
+            "grad_norm": norms.cpu().numpy(),
+            "grad_sample": bucket.flat[idx].cpu().numpy()}
+
+
+def write_outputs(out_dir, arrays):
+    import numpy as np
+
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
+
+
 # ------------------------------------------------------------------------------------------------
 # our CUDA path
 # ------------------------------------------------------------------------------------------------
@@ -532,8 +559,14 @@ def main_ours(args):
     if sampler:
         sampler.start()
     _lib.reset_launch_count()
-    ms_total = timed(lambda: step(wsem_d, wco_d), args.steps)
+    last_loss = [None]
+
+    def headline_step():
+        last_loss[0] = step(wsem_d, wco_d).detach()
+
+    ms_total = timed(headline_step, args.steps)
     launches = _lib.launch_count() / args.steps
+    outputs = last_step_outputs(last_loss[0], bucket) if args.dump_outputs and rank == 0 else None
 
     # ---- end to end: pinned host ids -> device, loss -> host, every step ----
     def e2e_step():
@@ -635,6 +668,8 @@ def main_ours(args):
                                               "(restatement of the reference's modules; /root/reference is absent on the GPU box)"}
         except Exception as e:  # pragma: no cover
             line["cpu_baseline"] = {"error": repr(e)}
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -648,7 +683,13 @@ if __name__ == "__main__":
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the bounded CPU baseline leg")
     ap.add_argument("--headline-only", action="store_true", help="skip the extra C1/C2/C4/C5 legs of the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss and gradients of the last timed step as DIR/<name>.npy (rank 0)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes what the CUDA path computed; it does not apply to --impl reference")
     # NCCL / torch may print banners ("NCCL version ...") on fd 1: keep stdout for the JSON line only
     sys.stdout.flush()
     _REAL_STDOUT = os.dup(1)

@@ -141,6 +141,32 @@ def test_flat_bucket_ranges():
     b.finish()
 
 
+def test_bench_dump_outputs_are_seeded_and_bounded(tmp_path):
+    """bench.py --dump-outputs: float32 / float64 .npy files, the same sample positions on every call, under 64 MB."""
+    import numpy as np
+
+    import bench
+    from audiolm_pytorch_b200.parallel import FlatGradBucket
+
+    m = torch.nn.Sequential(torch.nn.Linear(300, 200), torch.nn.Linear(200, 10))
+    b = FlatGradBucket(m.parameters())
+    b.flat.copy_(torch.arange(b.numel, dtype=torch.float32))
+    out = bench.last_step_outputs(torch.tensor(2.5), b)
+    bench.write_outputs(tmp_path / "a", out)
+    bench.write_outputs(tmp_path / "b", bench.last_step_outputs(torch.tensor(2.5), b))
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["grad_norm.npy", "grad_sample.npy", "loss.npy"]
+    for name in files:
+        a, c = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, c), name
+    assert float(np.load(tmp_path / "a" / "loss.npy")) == 2.5
+    sample = np.load(tmp_path / "a" / "grad_sample.npy")
+    assert np.array_equal(sample, np.sort(sample)) and sample.max() < b.numel   # positions of the flat gradient
+    norms = np.load(tmp_path / "a" / "grad_norm.npy")
+    assert np.allclose(norms, [p.grad.double().norm().item() for p in b.params])
+    assert bench.DUMP_GRAD_SAMPLES * 4 + 142 * 8 + 4 < 64 << 20   # the benchmarked model has 142 parameters
+
+
 def test_batch_unique_consecutive_matches_per_row_loop():
     """vectorised version vs the reference construction (audiolm_pytorch.py:162-164)"""
     from torch import nn
