@@ -37,8 +37,7 @@ SIGNATURES: dict[str, list] = {
     "alm_bias_gather_fwd": [P, P, P, P, I, I, I, L, P],
     "alm_bias_gather_bwd": [P, P, P, P, I, I, I, L, P],
     "alm_hc_pre_fwd": [P] * 12 + [P, P, P, P, P, I, I, I, P],
-    "alm_hc_pre_bwd": [P] * 12 + [P, P, P, P, P, P, P, P, P, F] + [P] * 8 + [P, P] + [I, I, I, P],
-    "alm_hc_param_finish": [P, P, P, P, P, P, P, I, P],
+    "alm_hc_pre_bwd": [P] * 12 + [P, P, P, P, P, P, P, P, P, F] + [P] * 8 + [P, I] + [I, I, I, P],
     "alm_hc_post_fwd": [P, P, P, P, P, P, I, I, I, P],
     "alm_hc_post_bwd": [P, P, P, P, P, P, P, P, P, P, I, I, I, P],
     "alm_geglu_ln_fwd": [P, L, I, P, P, L, P, I, I, I, P],

@@ -10,8 +10,7 @@
 // token contiguous; M = batch * seq.  One CTA walks tokens with a grid stride; thread t owns the 8
 // contiguous channels [8t, 8t+8) of every stream, so d/8 threads are active (d % 8 == 0, d <= 8192).
 #include "alm_common.cuh"
-#include "hyper_conn_v2.cuh"
-#include "hyper_conn_v3.cuh"
+#include "hyper_conn_v4.cuh"
 
 namespace alm {
 
@@ -75,7 +74,7 @@ __device__ __forceinline__ void load8f(const float* p, float (&f)[8]) {
 
 // Saved per token for the backward: tanh of the dynamic alpha/beta pre-activations, 1/|R_s|, LN stats.
 //   aux [M, AUX] = { ta[S*(S+1)], tb[S], inv_nrm[S], mean, rstd }
-constexpr int HC_AUX = HC_S * HC_T + HC_S + HC_S + (HC_S * HC_T + HC_S) + 2;  // same stride as hc2::AUX (z slots unused here)
+constexpr int HC_AUX = hc4::AUX;  // same stride as the d <= 1024 kernels (z slots unused here)
 
 // ---------------------------------------------------------------------------------------------
 // forward:  R = R_in + beta_prev (x) Y   (or R_s = x for every s when expanding)
@@ -659,17 +658,17 @@ extern "C" int alm_hc_pre_fwd(const void* R_in, const void* Y, const float* beta
   ALM_REQUIRE(streams == HC_S, ALM_ERR_UNSUPPORTED);
   ALM_REQUIRE(d % 8 == 0 && d >= 8 && d <= 8192 && M > 0, ALM_ERR_ARG);
   ALM_REQUIRE((x_expand != nullptr) != (R_in != nullptr), ALM_ERR_ARG);
-  if (d <= 1024) {  // second-generation kernel: 2 or 4 warps per token, no CTA-wide barriers
-    hc2::Params p2{gamma_hc, dyn_alpha, dyn_beta, static_alpha, static_beta, alpha_scale, beta_scale, ln_gamma};
-    const int tpt = 64;  // 4 warps per token (tpt 128) measured slower at d=1024: 297 vs 227 us
-    const int tok = hc2::THREADS / tpt;
-    const int grid = min(ceil_div(M, tok), num_sms() * 2);
-    const size_t smem = hc2::fwd_smem(d, tpt);
-#define HC2_FWD_ARGS (const __nv_bfloat16*)R_in, (const __nv_bfloat16*)Y, beta_prev, x_expand, p2, (__nv_bfloat16*)R_out, \
-                     (__nv_bfloat16*)bin, (__nv_bfloat16*)xn, beta_out, aux, M, d
-    if (d <= 512) hc2::pre_fwd_kernel<1, 64><<<grid, hc2::THREADS, smem, stream>>>(HC2_FWD_ARGS);
-    else hc2::pre_fwd_kernel<2, 64><<<grid, hc2::THREADS, smem, stream>>>(HC2_FWD_ARGS);
-#undef HC2_FWD_ARGS
+  if (d <= 1024) {
+    hc4::Params p4{gamma_hc, dyn_alpha, dyn_beta, static_alpha, static_beta, alpha_scale, beta_scale, ln_gamma};
+    const int grid = min(M, hc4::FWD_CTAS_PER_SM * num_sms());
+    const size_t smem = hc4::param_smem(d);
+    if (x_expand != nullptr)
+      hc4::pre_fwd_kernel<true><<<grid, hc4::THREADS, smem, stream>>>(nullptr, nullptr, nullptr, x_expand, p4,
+          (__nv_bfloat16*)R_out, (__nv_bfloat16*)bin, (__nv_bfloat16*)xn, beta_out, aux, M, d);
+    else
+      hc4::pre_fwd_kernel<false><<<grid, hc4::THREADS, smem, stream>>>((const __nv_bfloat16*)R_in,
+          (const __nv_bfloat16*)Y, beta_prev, nullptr, p4, (__nv_bfloat16*)R_out, (__nv_bfloat16*)bin,
+          (__nv_bfloat16*)xn, beta_out, aux, M, d);
     ALM_CHECK_LAUNCH();
     ALM_LAUNCHED(1);
     return ALM_OK;
@@ -691,67 +690,39 @@ extern "C" int alm_hc_pre_bwd(const void* R_in, const void* Y, const float* beta
                               const void* dxn, const void* dbin_extra, const float* dbeta, void* dR_in, void* dY,
                               float* dbeta_prev, float* dx_expand, float dx_scale, float* g_gamma_hc,
                               float* g_dyn_alpha, float* g_dyn_beta, float* g_static_alpha, float* g_static_beta,
-                              float* g_alpha_scale, float* g_beta_scale, float* g_ln_gamma, void* w_out,
-                              void* wy_out, int M, int d, int streams, alm_stream_t stream_) {
+                              float* g_alpha_scale, float* g_beta_scale, float* g_ln_gamma, float* partial,
+                              int partial_blocks, int M, int d, int streams, alm_stream_t stream_) {
   cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
   ALM_REQUIRE(streams == HC_S, ALM_ERR_UNSUPPORTED);
   ALM_REQUIRE(d % 8 == 0 && d >= 8 && d <= 8192 && M > 0, ALM_ERR_ARG);
-  ALM_REQUIRE((w_out == nullptr) == (wy_out == nullptr), ALM_ERR_ARG);
-  if (w_out != nullptr) {
-    // hc3: the per-channel parameter gradients are left to the caller (skinny GEMMs over w_out / wy_out)
-    ALM_REQUIRE(d <= 1024 && x_expand == nullptr && R_in != nullptr && Y != nullptr, ALM_ERR_UNSUPPORTED);
-    hc2::Params p3{gamma_hc, dyn_alpha, dyn_beta, static_alpha, static_beta, alpha_scale, beta_scale, ln_gamma};
-    hc2::Grads g3{g_gamma_hc, g_dyn_alpha, g_dyn_beta, g_static_alpha, g_static_beta, g_alpha_scale, g_beta_scale,
-                  g_ln_gamma};
-    const int nch = ceil_div(d, 256);
-    const size_t smem = hc3::bwd_smem(d);
-    static bool attr3 = false;
-    if (!attr3) {
-      ALM_CUDA_OK(cudaFuncSetAttribute(hc3::pre_bwd_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hc3::bwd_smem(256)));
-      ALM_CUDA_OK(cudaFuncSetAttribute(hc3::pre_bwd_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hc3::bwd_smem(512)));
-      ALM_CUDA_OK(cudaFuncSetAttribute(hc3::pre_bwd_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hc3::bwd_smem(768)));
-      ALM_CUDA_OK(cudaFuncSetAttribute(hc3::pre_bwd_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hc3::bwd_smem(1024)));
-      attr3 = true;
-    }
-    const int grid3 = min(ceil_div(M, hc3::TOK), 2 * num_sms());
-#define HC3_ARGS (const __nv_bfloat16*)R_in, (const __nv_bfloat16*)Y, beta_prev, p3, aux, (const __nv_bfloat16*)dR_out, \
-                 (const __nv_bfloat16*)dxn, (const __nv_bfloat16*)dbin_extra, dbeta, (__nv_bfloat16*)dR_in,             \
-                 (__nv_bfloat16*)dY, dbeta_prev, (__nv_bfloat16*)w_out, (__nv_bfloat16*)wy_out, g3, M, d
-    switch (nch) {
-      case 1: hc3::pre_bwd_kernel<1><<<grid3, hc3::THREADS, smem, stream>>>(HC3_ARGS); break;
-      case 2: hc3::pre_bwd_kernel<2><<<grid3, hc3::THREADS, smem, stream>>>(HC3_ARGS); break;
-      case 3: hc3::pre_bwd_kernel<3><<<grid3, hc3::THREADS, smem, stream>>>(HC3_ARGS); break;
-      default: hc3::pre_bwd_kernel<4><<<grid3, hc3::THREADS, smem, stream>>>(HC3_ARGS); break;
-    }
-#undef HC3_ARGS
-    ALM_CHECK_LAUNCH();
-    ALM_LAUNCHED(1);
-    return ALM_OK;
-  }
   if (d <= 1024) {
-    hc2::Params p2{gamma_hc, dyn_alpha, dyn_beta, static_alpha, static_beta, alpha_scale, beta_scale, ln_gamma};
-    hc2::Grads g2{g_gamma_hc, g_dyn_alpha, g_dyn_beta, g_static_alpha, g_static_beta, g_alpha_scale, g_beta_scale,
+    const int grid = min(min(M, hc4::BWD_CTAS_PER_SM * num_sms()), partial_blocks);
+    ALM_REQUIRE(partial != nullptr && grid > 0, ALM_ERR_ARG);
+    hc4::Params p4{gamma_hc, dyn_alpha, dyn_beta, static_alpha, static_beta, alpha_scale, beta_scale, ln_gamma};
+    hc4::Grads g4{g_gamma_hc, g_dyn_alpha, g_dyn_beta, g_static_alpha, g_static_beta, g_alpha_scale, g_beta_scale,
                   g_ln_gamma};
-    const int tpt = 64;  // tpt 128 (4 warps per token, 2 CTAs/SM, 128-register cap) measured slower: 883 vs 713 us
-    const int tok = hc2::THREADS / tpt;
-    const int grid2 = min(ceil_div(M, tok), num_sms());
-    const size_t smem = hc2::bwd_smem(d, tpt);
-    static bool attr_set = false;
-    if (!attr_set) {
-      ALM_CUDA_OK(cudaFuncSetAttribute(hc2::pre_bwd_kernel<1, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)hc2::bwd_smem(512, 64)));
-      ALM_CUDA_OK(cudaFuncSetAttribute(hc2::pre_bwd_kernel<2, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)hc2::bwd_smem(1024, 64)));
-      attr_set = true;
+    float* part_small = partial + (size_t)grid * d * 8;
+    const bool expand = x_expand != nullptr;
+    const size_t smem = hc4::bwd_smem(d, expand);
+    static bool attr4 = false;
+    if (!attr4) {
+      ALM_CUDA_OK(cudaFuncSetAttribute(hc4::pre_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)hc4::bwd_smem(1024, false)));
+      ALM_CUDA_OK(cudaFuncSetAttribute(hc4::pre_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)hc4::bwd_smem(1024, true)));
+      attr4 = true;
     }
-#define HC2_BWD_ARGS (const __nv_bfloat16*)R_in, (const __nv_bfloat16*)Y, beta_prev, x_expand, p2, aux,              \
-                     (const __nv_bfloat16*)dR_out, (const __nv_bfloat16*)dxn, (const __nv_bfloat16*)dbin_extra, dbeta, \
-                     (__nv_bfloat16*)dR_in, (__nv_bfloat16*)dY, dbeta_prev, dx_expand, dx_scale, g2, M, d
-    if (d <= 512) hc2::pre_bwd_kernel<1, 64><<<grid2, hc2::THREADS, smem, stream>>>(HC2_BWD_ARGS);
-    else hc2::pre_bwd_kernel<2, 64><<<grid2, hc2::THREADS, smem, stream>>>(HC2_BWD_ARGS);
-#undef HC2_BWD_ARGS
+#define HC4_BWD_ARGS (const __nv_bfloat16*)R_in, (const __nv_bfloat16*)Y, beta_prev, x_expand, p4, aux,          \
+                        (const __nv_bfloat16*)dR_out, (const __nv_bfloat16*)dxn, (const __nv_bfloat16*)dbin_extra, \
+                        dbeta, (__nv_bfloat16*)dR_in, (__nv_bfloat16*)dY, dbeta_prev, dx_expand, dx_scale, partial,  \
+                        part_small, M, d
+    if (expand) hc4::pre_bwd_kernel<true><<<grid, hc4::THREADS, smem, stream>>>(HC4_BWD_ARGS);
+    else hc4::pre_bwd_kernel<false><<<grid, hc4::THREADS, smem, stream>>>(HC4_BWD_ARGS);
+#undef HC4_BWD_ARGS
     ALM_CHECK_LAUNCH();
-    ALM_LAUNCHED(1);
+    hc4::param_finish_kernel<<<d / 4 + 1, hc4::FIN_WARPS * 32, 0, stream>>>(partial, part_small, grid, p4, g4, d);
+    ALM_CHECK_LAUNCH();
+    ALM_LAUNCHED(2);
     return ALM_OK;
   }
   HcParams prm{gamma_hc, dyn_alpha, dyn_beta, static_alpha, static_beta, alpha_scale, beta_scale, ln_gamma};
@@ -763,19 +734,6 @@ extern "C" int alm_hc_pre_bwd(const void* R_in, const void* Y, const float* beta
               (const __nv_bfloat16*)R_in, (const __nv_bfloat16*)Y, beta_prev, x_expand, prm, aux,
               (const __nv_bfloat16*)dR_out, (const __nv_bfloat16*)dxn, (const __nv_bfloat16*)dbin_extra, dbeta,
               (__nv_bfloat16*)dR_in, (__nv_bfloat16*)dY, dbeta_prev, dx_expand, dx_scale, gr, M, d);
-  ALM_CHECK_LAUNCH();
-  ALM_LAUNCHED(1);
-  return ALM_OK;
-}
-
-extern "C" int alm_hc_param_finish(const float* G, const float* gamma_hc, const float* dyn_alpha,
-                                   const float* dyn_beta, float* g_gamma_hc, float* g_dyn_alpha, float* g_dyn_beta,
-                                   int d, alm_stream_t stream_) {
-  cudaStream_t stream = reinterpret_cast<cudaStream_t>(stream_);
-  ALM_REQUIRE(G && gamma_hc && dyn_alpha && dyn_beta && g_gamma_hc && g_dyn_alpha && g_dyn_beta && d > 0, ALM_ERR_ARG);
-  hc2::Params p{gamma_hc, dyn_alpha, dyn_beta, nullptr, nullptr, nullptr, nullptr, nullptr};
-  hc2::Grads g{g_gamma_hc, g_dyn_alpha, g_dyn_beta, nullptr, nullptr, nullptr, nullptr, nullptr};
-  hc3::hc_param_finish_kernel<<<ceil_div(d, 128), 128, 0, stream>>>(G, p, g, d);
   ALM_CHECK_LAUNCH();
   ALM_LAUNCHED(1);
   return ALM_OK;

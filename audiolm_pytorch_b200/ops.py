@@ -5,6 +5,8 @@ stream.  No function has a CPU or stock-PyTorch implementation.
 """
 from __future__ import annotations
 
+import functools
+
 import torch
 
 from . import _lib
@@ -387,8 +389,12 @@ def bias_gather_bwd(dbias, idx, table_rows, *, want_override):
     return dtable, dover
 
 
-HC_BWD_SPLIT = True  # False: hc2 kernel with in-kernel parameter-gradient accumulators (kept for A/B tests)
 HC_AUX = 54  # floats of per-token state kept for the backward (see csrc/hyper_conn.cu)
+
+
+@functools.lru_cache(maxsize=None)
+def _sm_count(dev):
+    return torch.cuda.get_device_properties(dev).multi_processor_count
 
 
 def _hc_param_ptrs(hc, ln_gamma):
@@ -415,7 +421,8 @@ def hc_pre_fwd(hc, ln_gamma, *, R_in=None, Y=None, beta_prev=None, x_expand=None
 
 def hc_pre_bwd(hc, ln_gamma, grads, g_ln_gamma, aux, dR_out, dxn, dbeta, *, dbin_extra=None, R_in=None, Y=None,
                beta_prev=None, x_expand=None, dx_scale=1.0, M, d, streams=4):
-    """Backward of hc_pre_fwd.  `grads`: dict of fp32 accumulators shaped like `hc` (atomically added to).
+    """Backward of hc_pre_fwd.  `grads`: dict of fp32 accumulators shaped like `hc` (added to; for d <= 1024 in a
+    fixed order, so the parameter gradients are bitwise reproducible).
 
     Returns (dR_in, dY, dbeta_prev) or dx_expand [M,d] f32 when the op expanded the streams.
     """
@@ -428,26 +435,15 @@ def hc_pre_bwd(hc, ln_gamma, grads, g_ln_gamma, aux, dR_out, dxn, dbeta, *, dbin
         dR_in = torch.empty(M, streams, d, device=dev, dtype=bf16)
         dY = torch.empty(M, d, device=dev, dtype=bf16)
         dbp = torch.empty(M, streams, device=dev, dtype=f32)
-    # hc3 path: per-channel parameter gradients via two skinny tcgen05 GEMMs instead of in-kernel accumulators
-    split = x_expand is None and d <= 1024 and HC_BWD_SPLIT
-    w = torch.empty(M * streams, 8, device=dev, dtype=bf16) if split else None
-    wy = torch.empty(M, 8, device=dev, dtype=bf16) if split else None
+    # per-CTA parameter-gradient partial sums of the d <= 1024 kernel (at most 3 CTAs per SM), reduced in a fixed order
+    blocks = 3 * _sm_count(dev)
+    partial = torch.empty(blocks * (8 * d + 32), device=dev, dtype=f32) if d <= 1024 else None
     nbytes = M * d * ((4 + 8 + 2 + 4 if x_expand is not None else 8 + 2 + 8 + 2 + 8 + 2) + (2 if dbin_extra is not None else 0))
     with _timed("hc_pre_bwd", nbytes, "byte"):
         _lib.call("alm_hc_pre_bwd", R_in, Y, beta_prev, x_expand, *_hc_param_ptrs(hc, ln_gamma), aux, dR_out, dxn,
                   dbin_extra, dbeta, dR_in, dY, dbp, dx, float(dx_scale),
                   grads["gamma"], grads["dyn_alpha"], grads["dyn_beta"], grads["static_alpha"], grads["static_beta"],
-                  grads["alpha_scale"], grads["beta_scale"], g_ln_gamma, w, wy, M, d, streams)
-    if split:
-        G = torch.zeros(d, 8, device=dev, dtype=f32)
-        rows = M * streams
-        sk = max(1, min(64, (rows // 64) // 8, 2 * 148 // max(1, (d + 127) // 128)))
-        # (HBM-bound: they stream R_in / Y once; kept out of the tensor-bound GEMM class of the roofline)
-        gemm(R_in.view(rows, d), w, a_mn=True, b_mn=True, out=G, acc_mode=2, split_k=sk, cls="gemm_skinny_hc_param_grad")
-        sk = max(1, min(64, (M // 64) // 8, 2 * 148 // max(1, (d + 127) // 128)))
-        gemm(Y, wy, a_mn=True, b_mn=True, out=G, acc_mode=2, split_k=sk, cls="gemm_skinny_hc_param_grad")
-        _lib.call("alm_hc_param_finish", G, hc["gamma"], hc["dyn_alpha"], hc["dyn_beta"], grads["gamma"],
-                  grads["dyn_alpha"], grads["dyn_beta"], d)
+                  grads["alpha_scale"], grads["beta_scale"], g_ln_gamma, partial, blocks, M, d, streams)
     return dx if x_expand is not None else (dR_in, dY, dbp)
 
 

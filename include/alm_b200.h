@@ -208,16 +208,13 @@ int alm_hc_pre_bwd(const void* R_in, const void* Y, const float* beta_prev, cons
                    const void* dbin_extra, const float* dbeta, void* dR_in, void* dY, float* dbeta_prev,
                    float* dx_expand, float dx_scale, float* g_gamma_hc, float* g_dyn_alpha, float* g_dyn_beta,
                    float* g_static_alpha, float* g_static_beta, float* g_alpha_scale, float* g_beta_scale,
-                   float* g_ln_gamma, void* w_out, void* wy_out, int M, int d, int streams, alm_stream_t stream);
+                   float* g_ln_gamma, float* partial, int partial_blocks, int M, int d, int streams,
+                   alm_stream_t stream);
 /*
- * alm_hc_pre_bwd with w_out / wy_out (both or neither; d <= 1024, not the expand branch): the kernel leaves the
- * per-channel parameter gradients (gamma_hc, dyn_alpha, dyn_beta) to the caller and writes
- *   w_out [M*4, 8] bf16 = inv_s * dz[t,s,c] (c < 6, zero padded),  wy_out [M, 8] bf16 = sum_s beta_prev_s * w[t,s,:]
- * so that G [d, 8] = R_in^T w_out + Y^T wy_out (two skinny alm_gemm_bf16 calls, MN-major operands) and
- * alm_hc_param_finish adds  g_dyn_alpha += g1*G[:, :5], g_dyn_beta += g1*G[:,5], g_gamma_hc += sqrt(d)*sum_c P_c G_c.
+ * alm_hc_pre_bwd, d <= 1024: the per-channel parameter gradients are summed per CTA in fp32 into `partial`
+ * (room for partial_blocks * (8*d + 32) floats; the kernel runs at most partial_blocks CTAs) and reduced from there
+ * in a fixed order, so every parameter gradient is bitwise reproducible.  d > 1024 ignores `partial`.
  */
-int alm_hc_param_finish(const float* G, const float* gamma_hc, const float* dyn_alpha, const float* dyn_beta,
-                        float* g_gamma_hc, float* g_dyn_alpha, float* g_dyn_beta, int d, alm_stream_t stream);
 /* last depth connection + reduce_streams (sum) + final LayerNorm (audiolm_pytorch.py:551-555) */
 int alm_hc_post_fwd(const void* R_in, const void* Y, const float* beta_prev, const float* ln_gamma, void* out,
                     float* stats, int M, int d, int streams, alm_stream_t stream);

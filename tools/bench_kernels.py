@@ -67,10 +67,13 @@ if "hc" in which:
     def hcb():
         return ops.hc_pre_bwd(hc, lng, grads, gl, aux, dR, dxn, dbe, dbin_extra=dbin, R_in=R, Y=Y, beta_prev=bp, M=M, d=d)
 
-    timeit("hc_pre_bwd (+2 skinny gemm+finish)", hcb, nbytes=M * d * 32)
-    ops.HC_BWD_SPLIT = False
-    timeit("hc_pre_bwd hc2 (in-kernel pgrads)", hcb, nbytes=M * d * 32)
-    ops.HC_BWD_SPLIT = True
+    timeit("hc_pre_bwd (+ param finish)", hcb, nbytes=M * d * 32)
+    x = rnd(M, d, dt=f32)
+    timeit("hc_pre_fwd x_expand", lambda: ops.hc_pre_fwd(hc, lng, x_expand=x, M=M, d=d), nbytes=M * d * 16)
+    aux_x = ops.hc_pre_fwd(hc, lng, x_expand=x, M=M, d=d)[4]
+    timeit("hc_pre_bwd x_expand (+ param finish)",
+           lambda: ops.hc_pre_bwd(hc, lng, grads, gl, aux_x, dR, dxn, dbe, dbin_extra=dbin, x_expand=x, M=M, d=d),
+           nbytes=M * d * 20)
 
 if "attn" in which:
     q, k, v = rnd(16, 2048, 512), rnd(16, 2048, 64), rnd(16, 2048, 64)
